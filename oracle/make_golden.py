@@ -19,6 +19,9 @@ from gigapose_b200 import synth
 from . import port, ref_import, ref_run
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
+# intra-op threads the fixtures are recorded with: how torch splits fp32 reductions across threads changes their last
+# bits, so tests/test_oracle_golden.py runs the port with the same count
+GOLDEN_THREADS = 8
 
 RETRIEVAL_CASES = {
     # BASELINE.json configs[0]: single query vs 16 templates, 1 object
@@ -38,6 +41,20 @@ def input_checksums(case):
                 ck_bank_mask=checksum(case.bank_mask16), ck_q_mask=checksum(case.q_mask16))
 
 
+def write_reference_init_case(B=3, O=2, T=12, seed=5):
+    """The retrieval sequence with the reference's own seeded IST initialisation (`ref_run.build_ist`), not the port's
+    weights: the regressor is rebuilt from the seed by the test, checked by `ck_regressor`."""
+    case = synth.make_feature_case(B=B, O=O, T=T, seed=seed)
+    ist = ref_run.build_ist()
+    out = ref_run.retrieval(synth.to_reference_layout(case), ist)
+    arrays = {k: v.numpy() for k, v in out.items()}
+    arrays.update({k: np.float64(v) for k, v in input_checksums(case).items()})
+    arrays["ck_regressor"] = np.float64(sum(checksum(v) for v in ist.regressor.state_dict().values()))
+    arrays["cfg"] = np.array([B, O, T, seed, 0])
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "retrieval_reference_init.npz"), **arrays)
+    print("retrieval_reference_init", {k: v.shape for k, v in arrays.items() if v.ndim})
+
+
 def reference_ist_with_port_weights():
     ist = ref_run.build_ist()
     ist.regressor.load_state_dict(port.RegressorPort().state_dict())
@@ -46,7 +63,7 @@ def reference_ist_with_port_weights():
 
 
 def main():
-    torch.set_num_threads(max(1, os.cpu_count() or 1))
+    torch.set_num_threads(GOLDEN_THREADS)
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     ist = reference_ist_with_port_weights()
     for name, cfg in RETRIEVAL_CASES.items():
@@ -57,6 +74,7 @@ def main():
         arrays["cfg"] = np.array([cfg["B"], cfg["O"], cfg["T"], cfg["seed"], cfg["sub_batch"] or 0])
         np.savez_compressed(os.path.join(GOLDEN_DIR, name + ".npz"), **arrays)
         print(name, {k: v.shape for k, v in arrays.items() if hasattr(v, "shape") and v.ndim})
+    write_reference_init_case()
 
     # a1: reference AENet (ae_net.py:55-69) wrapping the seeded ViT restatement; a6: reference ResNet
     ns = ref_import.load()

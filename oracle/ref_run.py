@@ -1,5 +1,5 @@
 """TEST INFRASTRUCTURE ONLY -- drives the *unmodified reference modules* (oracle/ref_import.py) through the
-same sequence as GigaPose.eval_retrieval (gigaPose.py:497-604).  Build container only."""
+same sequence as GigaPose.eval_retrieval (gigaPose.py:497-604).  `retrieval` needs the reference tree."""
 from __future__ import annotations
 
 import pandas as pd
@@ -11,8 +11,11 @@ IST_CFG = dict(n_heads=0, input_dim=3, input_size=256, initial_dim=128, block_di
                descriptor_size=256)
 
 
-def build_ist(seed=8):
-    ns = ref_import.load()
+def build_ist(seed=8, classes=None):
+    """Seeded ISTNet of the reference's classes, or of `classes` (a namespace with ResNet, Regressor, ISTNet): this
+    repository's drop-in classes create and initialise their parameters in the reference's order, so the same seed
+    gives the same weights without a reference tree."""
+    ns = classes or ref_import.load()
     torch.manual_seed(seed)
     backbone = ns.ResNet(dict(IST_CFG))
     regressor = ns.Regressor(descriptor_size=256, hidden_dim=256, use_tanh_act=True, normalize_output=True)

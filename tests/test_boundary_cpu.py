@@ -1,20 +1,62 @@
 """CPU test of the drop-in boundary (SURVEY §8b, VERDICT r1 item 5): with this repository BEFORE a reference checkout on
 sys.path -- INTEGRATION.md's recipe -- every Hydra `_target_` of the reference's own model configs resolves to this
 repository's classes and instantiates with the YAML's own kwargs, while the modules outside the hot path that `test.py`
-needs (`src.dataloader.template`, `src.utils.bbox`, ...) still import from the checkout.  Skipped when /root/reference is
-absent (the GPU box)."""
+needs (`src.dataloader.template`, `src.utils.bbox`, ...) still import from the checkout.  The model configs are the
+reference's own, recorded in tests/golden/model_configs.json (`python -m oracle.make_golden_configs`); the checkout is a
+stand-in written by the test whose modules import the way the reference's do (see `_CHECKOUT`)."""
 import importlib
+import json
 import os
 import subprocess
 import sys
 import textwrap
 
-import pytest
-import yaml
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "configs")), reason="reference checkout not present")
+CONFIGS = os.path.join(ROOT, "tests", "golden", "model_configs.json")
+
+# Modules outside the hot path, laid out like a reference checkout (`src` and its sub-packages without __init__.py).
+# Their imports follow src/dataloader/template.py and src/custom_megapose/template_dataset.py of the reference: names from
+# files this repository also has (`src.utils.dataset`, `src.utils.logging`, `src.megapose.utils.tensor_collection`), a
+# name only the checkout's copy of such a file has (`src.utils.inout.combine`), modules only the checkout has inside
+# packages both have (`src.lib3d.numpy`, `src.utils.pil`) and packages only the checkout has.
+_CHECKOUT = {
+    "src/dataloader/template.py": """
+        import src.megapose.utils.tensor_collection as tc
+        from src.custom_megapose.template_dataset import NearestTemplateFinder, TemplateDataset
+        from src.utils.dataset import LMO_index_to_ID
+
+        class TemplateSet:
+            pass
+        """,
+    "src/custom_megapose/template_dataset.py": """
+        from src.custom_megapose.transform import Transform
+        from src.lib3d.numpy import R_opencv2R_opengl
+        from src.megapose.utils.tensor_collection import PandasTensorCollection
+        from src.utils.inout import combine
+        from src.utils.logging import get_logger
+        from src.utils.pil import open_image
+
+        class TemplateDataset:
+            pass
+
+        class NearestTemplateFinder:
+            pass
+        """,
+    "src/custom_megapose/transform.py": "class Transform:\n    pass\n",
+    "src/lib3d/numpy.py": "def R_opencv2R_opengl(R):\n    return R\n",
+    "src/utils/pil.py": "def open_image(path):\n    return path\n",
+    "src/utils/bbox.py": "def xyxy_to_xywh(box):\n    return box\n",
+    "src/utils/inout.py": "def combine(a, b):\n    return a + b\n",
+}
+
+
+def _write_checkout(root):
+    for rel, text in _CHECKOUT.items():
+        path = os.path.join(root, rel)
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        with open(path, "w") as f:
+            f.write(textwrap.dedent(text).lstrip())
+    return os.path.realpath(root)
 
 
 def _targets(node, out):
@@ -28,8 +70,10 @@ def _targets(node, out):
 
 def test_every_model_target_resolves_here():
     names = []
+    with open(CONFIGS) as f:
+        configs = json.load(f)
     for rel in ("model/large.yaml", "model/ae_net/dinov2_l.yaml", "model/ist_net/resnet.yaml"):
-        names += _targets(yaml.safe_load(open(os.path.join(REF, "configs", rel))), [])
+        names += _targets(configs[rel], [])
     assert "src.models.gigaPose.GigaPose" in names and "src.models.network.resnet.ResNet" in names
     for t in names:
         if t.startswith("torch."):
@@ -41,23 +85,9 @@ def test_every_model_target_resolves_here():
 
 
 _SCRIPT = r"""
-import os, sys, types, yaml
+import json, os, sys
 ROOT, REF = sys.argv[1], sys.argv[2]
 sys.path[:0] = [ROOT, REF, os.path.join(REF, "src")]     # INTEGRATION.md recipe (+ src/ for `import megapose...`)
-# third-party packages of the reference's environment that this container lacks (not part of either code base)
-for name in ("bop_toolkit_lib", "bop_toolkit_lib.inout", "bop_toolkit_lib.pycoco_utils", "pinocchio", "webdataset", "imageio"
-             ):
-    if name not in sys.modules:
-        try:
-            __import__(name)
-        except Exception:
-            m = types.ModuleType(name)
-            def _ga(attr):
-                if attr.startswith("__"):
-                    raise AttributeError(attr)
-                return type(attr, (), {})
-            m.__getattr__ = _ga
-            sys.modules[name] = m
 import importlib, torch
 import src
 assert any(p.startswith(REF) for p in src.__path__), src.__path__
@@ -73,8 +103,10 @@ def instantiate(node, **extra):
         return {k: instantiate(v) for k, v in node.items()}
     return node
 
+CONFIGS = json.load(open(sys.argv[4]))
+
 def load(rel):
-    return yaml.safe_load(open(os.path.join(REF, "configs", rel)))
+    return CONFIGS[rel]
 
 ae_cfg, ist_cfg, model_cfg = load("model/ae_net/dinov2_l.yaml"), load("model/ist_net/resnet.yaml"), load("model/large.yaml")
 ist_cfg["backbone"]["config"]["descriptor_size"] = ist_cfg["descriptor_size"]        # ${model.ist_net.descriptor_size}
@@ -112,6 +144,7 @@ print("BOUNDARY_OK")
 
 
 def test_reference_configs_instantiate_and_dataloaders_import(tmp_path):
-    r = subprocess.run([sys.executable, "-c", textwrap.dedent(_SCRIPT), ROOT, REF, str(tmp_path)], capture_output=True,
-                       text=True, timeout=600, cwd=str(tmp_path))
+    ref = _write_checkout(tmp_path / "checkout")
+    r = subprocess.run([sys.executable, "-c", textwrap.dedent(_SCRIPT), ROOT, ref, str(tmp_path), CONFIGS],
+                       capture_output=True, text=True, timeout=600, cwd=str(tmp_path))
     assert r.returncode == 0 and "BOUNDARY_OK" in r.stdout, r.stdout[-2000:] + r.stderr[-4000:]

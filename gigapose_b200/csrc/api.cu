@@ -8,7 +8,6 @@
 #include <dlfcn.h>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <new>
 #include <string>
@@ -86,15 +85,6 @@ int gp_internal_fail(int code, const char* fmt, ...) {
   return code;
 }
 void gp_internal_count_launches(int n) { g_launches += n; }
-namespace gp {
-// Off by default: a same-process A/B (scripts/pdl_ab.py, profiles/r02_pdl_ab.md) measured no gain on the ViT chain --
-// the persistent 1-CTA-per-SM kernels hold all shared memory / TMEM until they exit, so a dependent grid cannot become
-// resident early enough to hide anything but its own ~2 us prologue.  GIGAPOSE_PDL=1 turns it on (read at every launch).
-bool pdl_enabled() {
-  const char* ev = getenv("GIGAPOSE_PDL");
-  return ev ? (ev[0] != '0') : false;
-}
-}  // namespace gp
 
 // generic 2-D bf16 plane map [rows, cols] (cols contiguous) with explicit box and swizzle (64 or 128 = box_cols * 2 bytes)
 int gp_internal_make_map_ex(CUtensorMap* map, void* ptr, uint64_t rows, uint64_t cols, uint32_t box_cols, uint32_t box_rows,
@@ -149,10 +139,10 @@ int gp_internal_make_map(CUtensorMap* map, void* ptr, uint64_t rows, uint64_t co
 namespace {
 
 // k-block-tiled bf16 descriptor plane: [image][32 k-blocks][256 patches][32 channels]; seen by TMA as a 2-D array of
-// 64-byte rows [images * 32 * 256, 32]; box = 32 channels (64 B, SWIZZLE_64B) x box_rows patches of one k-block slab
-// (256 = all patches of a template, 128 = one t-half of a query)
-int make_plane_map(CUtensorMap* map, void* ptr, uint64_t images, uint32_t box_rows) {
-  return gp_internal_make_map_ex(map, ptr, images * 32ull * GP_NUM_PATCHES, 32, 32, box_rows, 64);
+// 64-byte rows [images * 32 * 256, 32]; box = 32 channels (64 B, SWIZZLE_64B) x 128 patches of one k-block slab (the
+// half of a query or template slab that one CTA of a similarity pair stages)
+int make_plane_map(CUtensorMap* map, void* ptr, uint64_t images) {
+  return gp_internal_make_map_ex(map, ptr, images * 32ull * GP_NUM_PATCHES, 32, 32, 128, 64);
 }
 
 struct Bank {
@@ -172,9 +162,11 @@ struct Workspace {
   uint8_t *rec_idx, *rec_valid;
   // local candidates
   float* c_score; int* c_id; float* c_pts_score; uint8_t *c_idx, *c_valid;
-  // IST MLP scratch (hidden1 / hidden2 double as the bf16 planes / per-head fp32 rows of the tensor-core form)
-  int* row_count; int* row_ids; float *hidden1, *hidden2;
-  uint16_t *mlp_a_hi, *mlp_a_lo;                       // gathered inputs [Bm*k*256, 512] as bf16 hi / lo planes
+  // IST MLP scratch: compacted valid rows and the activations of the two hidden layers
+  int* row_count; int* row_ids;
+  uint16_t *mlp_h1_hi, *mlp_h1_lo;                     // first hidden layer [Bm*k*256, 1024] as fp16 hi / lo planes
+  float *mlp_h2_scale, *mlp_h2_inplane;                // second hidden layer of each head [Bm*k*256, 256], fp32 rows
+  uint16_t *mlp_a_hi, *mlp_a_lo;                       // gathered inputs [Bm*k*256, 512] as fp16 hi / lo planes
   uint16_t *w1_hi, *w1_lo, *w2s_hi, *w2s_lo, *w2i_hi, *w2i_lo;   // packed regressor weights ([1024,512], [256,512] x 2)
   float* bias1;                                        // [1024] = scale b1 | inplane b1
 };
@@ -213,8 +205,10 @@ void carve_workspace(Carver& c, const gp_config_t& cfg, Workspace* w) {
   tmp.c_valid = c.take<uint8_t>(Bm * k * GP_NUM_PATCHES);
   tmp.row_count = c.take<int>(1);
   tmp.row_ids = c.take<int>(Bm * k * GP_NUM_PATCHES);
-  tmp.hidden1 = c.take<float>(Bm * k * GP_NUM_PATCHES * 1024);
-  tmp.hidden2 = c.take<float>(Bm * k * GP_NUM_PATCHES * 512);
+  tmp.mlp_h1_hi = c.take<uint16_t>(Bm * k * GP_NUM_PATCHES * 1024);
+  tmp.mlp_h1_lo = c.take<uint16_t>(Bm * k * GP_NUM_PATCHES * 1024);
+  tmp.mlp_h2_scale = c.take<float>(Bm * k * GP_NUM_PATCHES * 256);
+  tmp.mlp_h2_inplane = c.take<float>(Bm * k * GP_NUM_PATCHES * 256);
   tmp.mlp_a_hi = c.take<uint16_t>(Bm * k * GP_NUM_PATCHES * 512);
   tmp.mlp_a_lo = c.take<uint16_t>(Bm * k * GP_NUM_PATCHES * 512);
   tmp.w1_hi = c.take<uint16_t>(1024 * 512);
@@ -253,11 +247,8 @@ struct gp_context {
   Bank bank;
   Workspace ws;
   CUtensorMap tm_q_hi, tm_q_lo, tm_t_hi, tm_t_lo;
-  CUtensorMap tm_t_hi128, tm_t_lo128;   // 128-row boxes: each CTA of a pair stages half of a template slab
-  int sim_pair;      // similarity kernel on 2-CTA clusters (GIGAPOSE_SIM_PAIR, default on)
-  int mlp_tc;        // IST MLP hidden layers on tcgen05 (GIGAPOSE_MLP_SIMT=1 selects the fp32 SIMT kernels)
   CUtensorMap tm_ma_hi, tm_ma_lo;                 // MLP layer 1: gathered rows [rows,512]
-  CUtensorMap tm_h1s_hi, tm_h1s_lo, tm_h1i_hi, tm_h1i_lo;   // layer 2: column halves of hidden1 [rows,1024]
+  CUtensorMap tm_h1s_hi, tm_h1s_lo, tm_h1i_hi, tm_h1i_lo;   // layer 2: column halves of the first hidden layer [rows,1024]
   CUtensorMap tm_w1_hi, tm_w1_lo, tm_w2s_hi, tm_w2s_lo, tm_w2i_hi, tm_w2i_lo;
   gp::IstMlpWeights mlp;
   bool mlp_set;
@@ -326,14 +317,6 @@ int gp_create(const gp_config_t* cfg, void* bank_mem, void* workspace_mem, gp_ha
   h->num_sms = prop.multiProcessorCount;
   h->mlp_set = false;
   h->cur_B = 0;
-  {
-    const char* ev = getenv("GIGAPOSE_MLP_SIMT");
-    h->mlp_tc = ev ? (ev[0] == '0') : 1;
-  }
-  {
-    const char* ev = getenv("GIGAPOSE_SIM_PAIR");
-    h->sim_pair = ev ? (ev[0] != '0') : 1;      // default: the 2-CTA cluster kernel (GIGAPOSE_SIM_PAIR=0: 1-CTA kernel)
-  }
   h->nccl_comm = nullptr;
   h->rank = 0;
   h->world = 1;
@@ -343,16 +326,14 @@ int gp_create(const gp_config_t* cfg, void* bank_mem, void* workspace_mem, gp_ha
   const uint64_t bank_rows = (uint64_t)cfg->num_objects * cfg->num_templates;   // images
   const uint64_t q_rows = (uint64_t)cfg->max_batch;
   int e;
-  if ((e = make_plane_map(&h->tm_t_hi, h->bank.hi, bank_rows, 256)) || (e = make_plane_map(&h->tm_t_lo, h->bank.lo, bank_rows, 256)) ||
-      (e = make_plane_map(&h->tm_t_hi128, h->bank.hi, bank_rows, 128)) || (e = make_plane_map(&h->tm_t_lo128, h->bank.lo, bank_rows, 128)) ||
-      (e = make_plane_map(&h->tm_q_hi, h->ws.q_hi, q_rows, 128)) || (e = make_plane_map(&h->tm_q_lo, h->ws.q_lo, q_rows, 128))) {
+  if ((e = make_plane_map(&h->tm_t_hi, h->bank.hi, bank_rows)) || (e = make_plane_map(&h->tm_t_lo, h->bank.lo, bank_rows)) ||
+      (e = make_plane_map(&h->tm_q_hi, h->ws.q_hi, q_rows)) || (e = make_plane_map(&h->tm_q_lo, h->ws.q_lo, q_rows))) {
     delete h;
     return e;
   }
   {
     const uint64_t rows = (uint64_t)cfg->max_batch * cfg->top_k * GP_NUM_PATCHES;
-    uint16_t* h1_hi = reinterpret_cast<uint16_t*>(h->ws.hidden1);
-    uint16_t* h1_lo = h1_hi + rows * 1024;
+    uint16_t *h1_hi = h->ws.mlp_h1_hi, *h1_lo = h->ws.mlp_h1_lo;
     const uint64_t dims[2] = {512, rows}, strides[1] = {1024 * sizeof(uint16_t)};
     const uint32_t box[2] = {32, 128}, estr[2] = {1, 1};
     int e;
@@ -474,10 +455,10 @@ int gp_set_ist_weights(gp_handle_t h, const float* const w[12], int use_tanh, vo
   m.s_w1 = w[0]; m.s_b1 = w[1]; m.s_w2 = w[2]; m.s_b2 = w[3]; m.s_w3 = w[4]; m.s_b3 = w[5];
   m.i_w1 = w[6]; m.i_b1 = w[7]; m.i_w2 = w[8]; m.i_b2 = w[9]; m.i_w3 = w[10]; m.i_b3 = w[11];
   m.use_tanh = use_tanh;
-  // tensor-core form: both heads' first layers side by side as one [1024,512] operand, bf16 hi / lo planes
+  // both heads' first layers side by side as one [1024,512] operand, fp16 hi / lo planes
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   Workspace& ws = h->ws;
-  GP_CUDA(gp::launch_split_planes(w[0], 512, 512, 512, ws.w1_hi, ws.w1_lo, s, true, kMlpWeightScale));   // fp16 hi / lo (see gp_ist_mlp)
+  GP_CUDA(gp::launch_split_planes(w[0], 512, 512, 512, ws.w1_hi, ws.w1_lo, s, true, kMlpWeightScale));   // fp16 hi / lo (see ist_mlp.cu)
   GP_CUDA(gp::launch_split_planes(w[6], 512, 512, 512, ws.w1_hi + 512 * 512, ws.w1_lo + 512 * 512, s, true, kMlpWeightScale));
   GP_CUDA(gp::launch_split_planes(w[2], 256, 512, 512, ws.w2s_hi, ws.w2s_lo, s, true, kMlpWeightScale));
   GP_CUDA(gp::launch_split_planes(w[8], 256, 512, 512, ws.w2i_hi, ws.w2i_lo, s, true, kMlpWeightScale));
@@ -522,11 +503,7 @@ static int run_sim(gp_context* h, int B, cudaStream_t s, float* debug_tile = nul
   p.rec_idx = h->ws.rec_idx;
   p.rec_valid = h->ws.rec_valid;
   p.debug_tile = debug_tile;
-  p.pair = h->sim_pair;
-  if (p.pair)
-    GP_CUDA(gp::launch_sim_search(h->tm_q_hi, h->tm_q_lo, h->tm_t_hi128, h->tm_t_lo128, p, h->num_sms, s));
-  else
-    GP_CUDA(gp::launch_sim_search(h->tm_q_hi, h->tm_q_lo, h->tm_t_hi, h->tm_t_lo, p, h->num_sms, s));
+  GP_CUDA(gp::launch_sim_search(h->tm_q_hi, h->tm_q_lo, h->tm_t_hi, h->tm_t_lo, p, h->num_sms, s));
   g_launches += 1;
   return GP_OK;
 }
@@ -597,26 +574,14 @@ int gp_ist_mlp(gp_handle_t h, int b0, int n, const float* q_ist, int ist_layout,
   p.tar_pts = reinterpret_cast<const long long*>(m->tar_pts);
   p.q_obj = h->ws.q_obj + b0; p.q_ist = q_pm; p.bank_ist = h->bank.ist;
   p.rel_scale = rel_scale; p.rel_inplane = rel_inplane;
-  p.row_count = h->ws.row_count; p.row_ids = h->ws.row_ids; p.hidden1 = h->ws.hidden1; p.hidden2 = h->ws.hidden2;
-  if (!h->mlp_tc) {
-    GP_CUDA(gp::launch_ist_mlp(h->mlp, p, s));
-    g_launches += 4;
-    return GP_OK;
-  }
-  // tensor-core form: compacted valid rows (device-side count, no host sync) -> 512 -> [512 | 512] -> 256 + 256 -> heads.
-  // Operands are IEEE fp16 hi / lo pairs (not bf16): descriptors, weights and hidden activations of this regressor are
-  // O(1e-2 .. 1e2), where an fp16 pair carries 22 significant bits -- the regressor outputs then agree with the fp32 SIMT
-  // kernels to 2e-5 (bf16 pairs: 4e-5, which moved a pose component by 1.2e-3 on the parity suite), at the same tensor rate.
+  p.row_count = h->ws.row_count; p.row_ids = h->ws.row_ids;
+  // compacted valid rows (device-side count, no host sync) -> 512 -> [512 | 512] -> 256 + 256 -> heads (ist_mlp.cu)
   const int rows = n * c.top_k * GP_NUM_PATCHES;                      // a multiple of 256: whole pair tiles
-  const uint64_t max_rows = (uint64_t)c.max_batch * c.top_k * GP_NUM_PATCHES;
-  uint16_t* h1_hi = reinterpret_cast<uint16_t*>(h->ws.hidden1);
-  uint16_t* h1_lo = h1_hi + max_rows * 1024;
-  float* h2s = h->ws.hidden2;
-  float* h2i = h->ws.hidden2 + max_rows * 256;
+  float *h2s = h->ws.mlp_h2_scale, *h2i = h->ws.mlp_h2_inplane;
   GP_CUDA(gp::launch_mlp_gather_planes(p, h->ws.mlp_a_hi, h->ws.mlp_a_lo, s));
   gp::GemmParams g{};
   g.passes = 3; g.pair = 1; g.f16 = 1; g.acc_scale = 1.0f / kMlpWeightScale; g.m_dev = h->ws.row_count;
-  g.M = rows; g.N = 1024; g.K = 512; g.mode = gp::GEMM_PLANES_RELU; g.bias = h->ws.bias1; g.out_hi = h1_hi; g.out_lo = h1_lo;
+  g.M = rows; g.N = 1024; g.K = 512; g.mode = gp::GEMM_PLANES_RELU; g.bias = h->ws.bias1; g.out_hi = h->ws.mlp_h1_hi; g.out_lo = h->ws.mlp_h1_lo;
   GP_CUDA(gp::launch_vit_gemm(h->tm_ma_hi, h->tm_ma_lo, h->tm_w1_hi, h->tm_w1_lo, g, h->num_sms, s));
   g = gp::GemmParams{};
   g.passes = 3; g.pair = 1; g.f16 = 1; g.acc_scale = 1.0f / kMlpWeightScale; g.m_dev = h->ws.row_count;

@@ -307,14 +307,6 @@ __device__ __forceinline__ void tmem_st_32x16(uint32_t taddr, const uint32_t (&r
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
-// Programmatic dependent launch: a kernel launched with cudaLaunchAttributeProgrammaticStreamSerialization may become
-// resident while its predecessor in the stream is still running (its CTAs take SMs as the predecessor's CTAs retire and
-// run their prologue: barrier init, TMEM allocation, descriptor prefetch).  `pdl_wait` blocks until the predecessor grid
-// has completed and its writes are visible -- it must precede the first access to anything an earlier kernel wrote (and
-// the first write to anything an earlier kernel reads); it is a no-op for a normally launched kernel.
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
 __device__ __forceinline__ void named_barrier_sync(uint32_t id, uint32_t nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }

@@ -6,27 +6,16 @@
 
 namespace gp {
 
-// Launch helper shared by the .cu files: optional 2-CTA cluster and optional programmatic dependent launch
-// (GIGAPOSE_PDL=0 turns the latter off; kernels launched this way call pdl_wait() before touching earlier kernels' data).
-bool pdl_enabled();
+// Launch helper shared by the .cu files: cluster_x > 1 groups the CTAs into clusters of cluster_x along x.
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_ex(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, int cluster_x,
-                             bool pdl, Args&&... args) {
+                             Args&&... args) {
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  int na = 0;
-  if (cluster_x > 1) {
-    attr[na].id = cudaLaunchAttributeClusterDimension;
-    attr[na].val.clusterDim.x = cluster_x; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  if (pdl && pdl_enabled()) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
-    ++na;
-  }
-  cfg.attrs = attr; cfg.numAttrs = na;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeClusterDimension;
+  attr.val.clusterDim.x = cluster_x; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
+  cfg.attrs = &attr; cfg.numAttrs = cluster_x > 1 ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
@@ -47,8 +36,8 @@ struct SimSearchParams {
   uint8_t* rec_idx;           // [B,T,256]  idx_tar2src
   uint8_t* rec_valid;         // [B,T,256]  mask_all != 0
   float* debug_tile;          // nullable [num_items,256,256]: raw fp32 similarity tiles (tests only)
-  int pair;                   // 1: 2-CTA cluster kernel (cta_group::2, one item per pair; template maps with 128-row boxes)
 };
+// 2-CTA cluster kernel (cta_group::2, one item per pair): every TMA box is 128 rows, the template maps included
 cudaError_t launch_sim_search(const CUtensorMap& q_hi, const CUtensorMap& q_lo, const CUtensorMap& t_hi,
                               const CUtensorMap& t_lo, const SimSearchParams& p, int num_sms, cudaStream_t stream);
 int sim_search_smem_bytes();
@@ -125,11 +114,8 @@ struct IstMlpParams {
   // workspace
   int* row_count;             // [1]
   int* row_ids;               // [B*k*256] flat (b,k,t) of valid rows
-  float* hidden1;             // [B*k*256, 1024]
-  float* hidden2;             // [B*k*256, 512]
 };
-cudaError_t launch_ist_mlp(const IstMlpWeights& w, const IstMlpParams& p, cudaStream_t stream);
-// Tensor-core form of the two hidden layers (vit_gemm_kernel on bf16 hi/lo planes, fp32-faithful 3-pass products):
+// The two hidden layers run on tensor cores (vit_gemm_kernel on fp16 hi/lo planes, fp32-faithful 3-pass products):
 //  * compact (device-side, no host round trip) + gather: row r = cat(query IST descriptor at tar_pt, template IST descriptor
 //    at src_pt) of the r-th valid correspondence -> planes [rows, 512]; *p.row_count rows, the GEMMs read that count
 //    on the device (GemmParams::m_dev);

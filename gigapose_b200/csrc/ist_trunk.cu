@@ -12,11 +12,12 @@
 // pixel 2*xo - 4 (16-byte row pitch, 64-byte rows), so that one k-block is one filter row ky (K = 7 x 32 = 224 with
 // zero filter entries for the 8th pixel and the 4th channel).
 // ReLU, the residual add and the hi/lo split of the next layer's input are the GEMM epilogue.
+// The trunk runs on 1-CTA tiles: 2-CTA cluster tiles, which gain 3 % on the ViT linears, were measured 3 % slower here on
+// a B200 (96-row filter boxes for the 192-channel layers, 64 pair tiles on 74 clusters in layer4).
 #include "../../include/gigapose_b200.h"
 #include "gigapose_kernels.h"
 
 #include <cuda_bf16.h>
-#include <cstdlib>
 #include <new>
 #include <vector>
 
@@ -145,7 +146,6 @@ __global__ void merge_planes_kernel(const __nv_bfloat16* __restrict__ hi, const 
 
 struct gp_ist_trunk_context {
   int max_crops, passes, num_sms;
-  int pair;                    // non-swapped layers run as 2-CTA cluster tiles (tcgen05 cta_group::2)
   std::vector<Conv> convs;
   Planes act[4];               // NHWC activation planes, each sized for the largest map [max_crops,128,128,128]
   Planes stem;                 // [max_crops, 262, 264, 4] zero-bordered resized crops (NHWC4)
@@ -187,7 +187,6 @@ int run(gp_ist_trunk_context* h, int n, const float* crops, float* feat, int sto
     g.passes = h->passes; g.mode = c.mode; g.bn = c.bn;
     g.M = n * c.hout * c.hout; g.N = c.cout; g.K = c.Kpad;
     if (c.swap) { g.swap = 1; g.M = c.cout; g.N = n * c.hout * c.hout; }
-    else g.pair = h->pair;
     g.bias = c.bias ? c.bias : h->zero_bias;
     if (c.out_buf >= 0) { g.out_hi = h->act[c.out_buf].hi; g.out_lo = h->act[c.out_buf].lo; }
     else g.x = feat;
@@ -246,12 +245,6 @@ int gp_ist_trunk_create(int device, int max_crops, int precision, const gp_conv_
   if (!h) return gp_internal_fail(GP_ERR_INVALID, "out of host memory");
   h->max_crops = max_crops; h->num_sms = prop.multiProcessorCount;
   h->passes = precision == GP_PRECISION_FP32_SPLIT ? 3 : 1;
-  {
-    // measured on B200: pairs gain 3 % on the ViT linears but lose 3 % here (96-row filter boxes for the 192-channel
-    // layers, 64 pair tiles on 74 clusters in layer4), so the trunk keeps 1-CTA tiles unless asked
-    const char* ev = getenv("GIGAPOSE_CONV_PAIR");
-    h->pair = ev ? (ev[0] != '0') : 0;
-  }
   h->convs = make_schedule();
   Carver cw(weight_mem), cs(workspace_mem);
   carve_weights(cw, h, h->convs);
@@ -275,8 +268,8 @@ int gp_ist_trunk_create(int device, int max_crops, int precision, const gp_conv_
       ce = gp::launch_split_planes(w[i].weight, c.cout, c.K, c.Kpad, c.w.hi, c.w.lo, s);
     }
     if (ce != cudaSuccess) break;
-    // rows per TMA box: filters (a CTA of a pair stages half of the bn filter rows) / pixels
-    const uint32_t wbox = c.swap ? 128 : (h->pair ? c.bn / 2 : c.bn), pix_tile = c.swap ? 256 : 128;
+    // rows per TMA box: filters / pixels
+    const uint32_t wbox = c.swap ? 128 : c.bn, pix_tile = c.swap ? 256 : 128;
     if ((e = gp_internal_make_map(&c.w_hi, c.w.hi, c.cout, c.Kpad, wbox)) || (e = gp_internal_make_map(&c.w_lo, c.w.lo, c.cout, c.Kpad, wbox)))
       break;
     if (c.in_buf < 0) {

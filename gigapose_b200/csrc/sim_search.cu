@@ -1,18 +1,27 @@
 // Fused query<->template patch-similarity search for sm_100a (row a4 of SURVEY.md §8; replaces
 // LocalSimilarity.test, reference src/models/matching.py:188-316 with helpers :63-113).
 //
-// One work item = one (query b, template n) pair = one 256(t) x 256(s) x 1024(c) similarity tile.
-// A persistent CTA per SM walks the item list:
-//   warp 0   : TMA producer  -- streams K-blocks of the query / template descriptor planes into a 4-stage smem ring
-//   warp 1   : UMMA issuer   -- tcgen05.mma (cta_group::1, M=128, N=256, K=16, bf16 -> fp32) into TMEM; the two
-//                               t-halves of a tile run back to back into alternating 256-column accumulators, so
-//                               the epilogue of one half overlaps the tensor work of the next
+// One work item = one (query b, template n) pair = one 256(t) x 256(s) x 1024(c) similarity tile, computed by a 2-CTA
+// cluster on the two SMs of a TPC as ONE M=256 x N=256 UMMA stream (tcgen05 cta_group::2).  CTA r of the pair owns the
+// query rows t in [128r, 128r+128) and stages HALF of the template slab (s rows [128r, 128r+128)); the leader issues the
+// instructions, which read both CTAs' shared memory, and every CTA drains its own 128 accumulator rows.  Persistent
+// pairs walk the item list:
+//   warp 0   : TMA producer  -- streams K-blocks of the query / template descriptor planes into a 6-stage smem ring
+//   warp 1   : UMMA issuer   -- leader only: tcgen05.mma (cta_group::2, M=256, N=256, K=16, bf16 -> fp32) into TMEM;
+//                               consecutive items alternate between two 256-column accumulators, so the epilogue of one
+//                               item overlaps the tensor work of the next
 //   warp 2   : TMEM allocator
 //   warps 4-11: epilogue     -- tcgen05.ld the fp32 tile, apply masks + threshold (matching.py:234-236), row
 //                               max/arg-max (t->s) in registers, column max/arg-max (s->t) with redux.sync +
 //                               ballot, cycle-consistency / validity masks (matching.py:80-113,247-271) and the
 //                               per-template score (matching.py:274-278).  The [B,N,256,256] similarity tensor
 //                               never reaches HBM; per item only a 1.5 KB record + one float are written.
+// The column maxima (idx_src2tar: arg-max over ALL 256 query patches) of the two halves are exchanged through
+// distributed shared memory (st.shared::cluster + mbarrier release / acquire at cluster scope); the leader sums the
+// per-template score in ascending-t warp order.
+// Against a 1-CTA form (M = 128, the two t-halves of a tile back to back) the template planes are streamed from L2 / HBM
+// once per item instead of once per t-half, and each SM's tensor core reads 4 KB + 4 KB of operands per instruction
+// instead of 4 KB + 8 KB; that form was measured slower at both precisions and removed (profiles/r02_stress_c5shard.json).
 //
 // Precision: descriptors are stored as two bf16 planes (hi = bf16(x), lo = bf16(x - hi)); the tile is accumulated
 // as hi*hi + hi*lo + lo*hi in fp32 (3 tensor-core passes, ~2^-17 relative operand error), so the thresholded /
@@ -30,17 +39,13 @@ constexpr int kP = 256;                         // patches per crop (16 x 16)
 constexpr int kC = 1024;                        // descriptor channels
 constexpr int kBlockK = 32;                     // bf16 elements per stage row: 64 B = SWIZZLE_64B span
 constexpr int kRowBytes = kBlockK * 2;
-constexpr int kStages = 4;
-constexpr int kHalfRows = 128;                  // t-rows per UMMA (M = 128)
-constexpr int kQPlaneBytes = kHalfRows * kRowBytes;   // 8 KB : 128 query rows x 64 B
-constexpr int kTPlaneBytes = kP * kRowBytes;          // 16 KB: 256 template rows x 64 B
-constexpr int kStageBytes = 2 * kQPlaneBytes + 2 * kTPlaneBytes;   // q_hi, q_lo, t_hi, t_lo = 48 KB
+constexpr int kHalfRows = 128;                  // t-rows per CTA of a pair
+constexpr int kQPlaneBytes = kHalfRows * kRowBytes;   // 8 KB : 128 rows x 64 B
 constexpr int kNumKBlocks = kC / kBlockK;       // 32
 constexpr int kEpiWarps = 8;
 constexpr int kEpiThreads = kEpiWarps * 32;     // 256
 constexpr int kThreads = 4 * 32 + kEpiThreads;  // 384
 constexpr int kTmemCols = 512;                  // two 128 x 256 fp32 accumulators (double buffered)
-constexpr uint32_t kIdesc = umma_idesc_f16(128, 256, /*bf16*/ 1);
 
 // Item order: queries (sorted by object) are taken in chunks of kQueryChunk; inside a chunk the template index is the
 // outer loop.  CTAs that run together then share template tiles (queries of one object are adjacent) AND touch at
@@ -56,277 +61,6 @@ __device__ __forceinline__ void decode_item(int item, int B, int T, int& j, int&
   j = q0 + (r - n * qc);
 }
 
-struct __align__(8) SimSmemTail {
-  float smask[kP];                              // template mask sampled at 16x16 (float: alpha masks are not binary)
-  float tmask[kP];                              // query mask sampled at 16x16
-  float pmax[kEpiWarps][kP];                    // partial column max per group of 32 t-rows (group = t / 32)
-  float cmax[kP];                               // score_src2tar
-  float rmax_s[kP];                             // score_tar2src
-  float rowp_max[2][2][kHalfRows];              // [t-half][column half][row]: partial row maxima
-  float red[2][kEpiWarps];
-  uint8_t pidx[kEpiWarps][kP];
-  uint8_t cidx[kP];                             // idx_src2tar
-  uint8_t ridx_s[kP];                           // idx_tar2src
-  uint8_t rowp_idx[2][2][kHalfRows];
-  uint64_t full_bar[kStages];
-  uint64_t empty_bar[kStages];
-  uint64_t tmem_full_bar[2];
-  uint64_t tmem_empty_bar[2];
-  uint32_t tmem_base;
-};
-
-constexpr int kSmemBytes = 1024 /*alignment slack*/ + kStages * kStageBytes + sizeof(SimSmemTail);
-
-}  // namespace
-
-// Work unit of the producer / UMMA warps: (item, t-half) = a 128(t) x 256(s) x 1024(c) half tile.  The two halves of
-// a tile run back to back into alternating TMEM accumulators, so the epilogue of one half overlaps the tensor work
-// of the next (the template planes are streamed once per half: L2 -> SM traffic is not the limiter, see profiles/).
-template <bool kDebug>
-__global__ void __launch_bounds__(kThreads, 1)
-sim_search_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid_constant__ CUtensorMap tm_q_lo,
-                  const __grid_constant__ CUtensorMap tm_t_hi, const __grid_constant__ CUtensorMap tm_t_lo,
-                  SimSearchParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  // SWIZZLE_64B atoms repeat every 512 B; keep every plane 1024 B aligned
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  SimSmemTail& tail = *reinterpret_cast<SimSmemTail*>(smem + kStages * kStageBytes);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int passes = p.passes;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < kStages; ++s) {
-      mbar_init(&tail.full_bar[s], 1);
-      mbar_init(&tail.empty_bar[s], 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(&tail.tmem_full_bar[a], 1);
-      mbar_init(&tail.tmem_empty_bar[a], kEpiWarps);
-    }
-    fence_barrier_init();
-  }
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tm_q_hi);
-    tma_prefetch_desc(&tm_t_hi);
-    if (passes == 3) {
-      tma_prefetch_desc(&tm_q_lo);
-      tma_prefetch_desc(&tm_t_lo);
-    }
-  }
-  if (warp == 2) tmem_alloc(&tail.tmem_base, kTmemCols);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = tail.tmem_base;
-
-  if (warp == 0) {
-    // ======================================= TMA producer =======================================
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      const uint32_t tx_bytes = (passes == 3 ? 2 : 1) * (kQPlaneBytes + kTPlaneBytes);
-      for (int item = blockIdx.x; item < p.num_items; item += gridDim.x) {
-        int j, n;
-        decode_item(item, p.B, p.T, j, n);
-        const int b = p.perm[j];
-        const int t_img = p.q_obj[b] * p.T + n;
-        for (int half = 0; half < 2; ++half) {
-          for (int kbi = 0; kbi < kNumKBlocks; ++kbi) {
-            // the second t-half walks K backwards: the template slabs it needs first are the ones the first half
-            // touched last, i.e. the ones most likely still in L2 when nothing else shares the template (B_o = 1)
-            const int kb = half == 0 ? kbi : kNumKBlocks - 1 - kbi;
-            mbar_wait(&tail.empty_bar[stage], phase ^ 1);
-            uint8_t* st = smem + stage * kStageBytes;
-            mbar_arrive_expect_tx(&tail.full_bar[stage], tx_bytes);
-            // k-block-tiled planes: slab (image, kb) = 256 contiguous 64-byte rows
-            const int q_row = (b * kNumKBlocks + kb) * kP + half * kHalfRows;
-            const int t_row = (t_img * kNumKBlocks + kb) * kP;
-            tma_load_2d(st, &tm_q_hi, &tail.full_bar[stage], 0, q_row);
-            tma_load_2d(st + 2 * kQPlaneBytes, &tm_t_hi, &tail.full_bar[stage], 0, t_row);
-            if (passes == 3) {
-              tma_load_2d(st + 2 * kQPlaneBytes + kTPlaneBytes, &tm_t_lo, &tail.full_bar[stage], 0, t_row);
-              tma_load_2d(st + kQPlaneBytes, &tm_q_lo, &tail.full_bar[stage], 0, q_row);
-            }
-            if (++stage == kStages) { stage = 0; phase ^= 1; }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ======================================= UMMA issuer ========================================
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      uint32_t unit = 0;                                          // running half-tile counter
-      for (int item = blockIdx.x; item < p.num_items; item += gridDim.x) {
-        for (int half = 0; half < 2; ++half, ++unit) {
-          const uint32_t acc = unit & 1u;
-          mbar_wait(&tail.tmem_empty_bar[acc], ((unit >> 1) & 1u) ^ 1u);   // epilogue drained this accumulator
-          tc_fence_after();
-          const uint32_t d = tmem_base + acc * 256;
-          for (int kb = 0; kb < kNumKBlocks; ++kb) {
-            mbar_wait(&tail.full_bar[stage], phase);
-            tc_fence_after();
-            const uint32_t st = smem_u32(smem + stage * kStageBytes);
-            const uint32_t q_hi = st, q_lo = st + kQPlaneBytes, t_hi = st + 2 * kQPlaneBytes,
-                           t_lo = st + 2 * kQPlaneBytes + kTPlaneBytes;
-#pragma unroll
-            for (int pass = 0; pass < 3; ++pass) {
-              if (pass < passes) {
-                const uint32_t a = (pass == 2 ? q_lo : q_hi);
-                const uint32_t bsm = (pass == 1 ? t_lo : t_hi);
-#pragma unroll
-                for (int k16 = 0; k16 < kBlockK / 16; ++k16) {
-                  const uint32_t accum = (kb | pass | k16) != 0 ? 1u : 0u;
-                  umma_f16(d, umma_desc_kmajor<kRowBytes>(a + k16 * 32), umma_desc_kmajor<kRowBytes>(bsm + k16 * 32),
-                           kIdesc, accum);
-                }
-              }
-            }
-            umma_commit(&tail.empty_bar[stage]);                  // frees the smem stage once these MMAs retire
-            if (++stage == kStages) { stage = 0; phase ^= 1; }
-          }
-          umma_commit(&tail.tmem_full_bar[acc]);                  // accumulator complete -> epilogue
-        }
-      }
-    }
-  } else if (warp >= 4) {
-    // ========================================= epilogue =========================================
-    // warp e: TMEM lane quarter q = e % 4 (rows 32q..32q+31 of the half tile), column half ch = e / 4.
-    const int e = warp - 4;
-    const int q = e & 3, ch = e >> 2;
-    const int tid = e * 32 + lane;           // 0..255: also "patch owned by this thread" in the per-tile tail
-    const int r = q * 32 + lane;             // row within the half tile
-    const float thr = p.sim_threshold;
-    uint32_t unit = 0;
-    for (int item = blockIdx.x; item < p.num_items; item += gridDim.x) {
-      int j, n;
-      decode_item(item, p.B, p.T, j, n);
-      const int b = p.perm[j];
-      const size_t rec = (size_t)b * p.T + n;
-      tail.smask[tid] = p.bank_mask[((size_t)p.q_obj[b] * p.T + n) * kP + tid];
-      tail.tmask[tid] = p.q_mask[(size_t)b * kP + tid];
-      named_barrier_sync(1, kEpiThreads);
-
-      for (int half = 0; half < 2; ++half, ++unit) {
-        const uint32_t acc = unit & 1u;
-        const int t = half * kHalfRows + r;                     // query patch of this thread's row
-        const float tm = tail.tmask[t];
-        const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * 256 + ch * 128;
-        mbar_wait(&tail.tmem_full_bar[acc], (unit >> 1) & 1u);
-        tc_fence_after();
-        float rmax = -1.0f;                  // all candidates are >= 0 after thresholding -> first max wins
-        int ridx = 0;
-#pragma unroll 1
-        for (int c0 = 0; c0 < 128; c0 += 32) {
-          uint32_t v32[32];
-          tmem_ld_32x32(taddr + c0, v32);
-          tmem_ld_wait();
-          const int s0 = ch * 128 + c0;
-          uint32_t keep_m = 0, keep_b = 1;
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            if (kDebug) p.debug_tile[((size_t)item * kP + t) * kP + s0 + j] = __uint_as_float(v32[j]);
-            float v = __uint_as_float(v32[j]) * tail.smask[s0 + j];          // matching.py:234
-            v = v * tm;                                                       // matching.py:235
-            v = (v < thr) ? 0.0f : v;                                         // matching.py:236
-            if (v > rmax) { rmax = v; ridx = s0 + j; }                        // torch.max(dim=3): first maximum
-            const uint32_t bits = __float_as_uint(v);                         // v >= 0: float order == uint order
-            const uint32_t m = __reduce_max_sync(0xffffffffu, bits);
-            const uint32_t bal = __ballot_sync(0xffffffffu, bits == m);
-            if (lane == j) { keep_m = m; keep_b = bal; }                      // lane j keeps column s0 + j
-          }
-          const int g = half * 4 + q;                                         // group of 32 t-rows: t / 32
-          tail.pmax[g][s0 + lane] = __uint_as_float(keep_m);
-          tail.pidx[g][s0 + lane] = (uint8_t)(g * 32 + __ffs(keep_b) - 1);   // torch.max(dim=2): first maximum
-        }
-        tail.rowp_max[half][ch][r] = rmax;
-        tail.rowp_idx[half][ch][r] = (uint8_t)ridx;
-        // accumulator fully read: hand it back to the UMMA warp before the smem-only part
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&tail.tmem_empty_bar[acc]);
-        named_barrier_sync(1, kEpiThreads);
-        if (ch == 0) {                        // merge the two column halves of row r (ties: lower s wins)
-          float a = tail.rowp_max[half][0][r];
-          uint8_t ai = tail.rowp_idx[half][0][r];
-          const float c = tail.rowp_max[half][1][r];
-          if (c > a) { a = c; ai = tail.rowp_idx[half][1][r]; }
-          tail.rmax_s[t] = a;
-          tail.ridx_s[t] = ai;
-        }
-      }
-
-      {  // combine the 8 partial column maxima in ascending-t order (strict > keeps the first maximum)
-        float best = tail.pmax[0][tid];
-        uint8_t bi = tail.pidx[0][tid];
-#pragma unroll
-        for (int g = 1; g < kEpiWarps; ++g) {
-          const float v = tail.pmax[g][tid];
-          if (v > best) { best = v; bi = tail.pidx[g][tid]; }
-        }
-        tail.cmax[tid] = best;
-        tail.cidx[tid] = bi;
-      }
-      named_barrier_sync(1, kEpiThreads);
-
-      // matching.py:247-271 for query patch t = tid
-      const int t = tid;
-      const float rmax = tail.rmax_s[t];
-      const int ridx = tail.ridx_s[t];
-      const float tm = tail.tmask[t];
-      const bool mask_sim = rmax >= thr;
-      const int back = tail.cidx[ridx];                                   // idx_src2tar[idx_tar2src[t]]
-      const float dx = (float)(back & 15) - (float)(t & 15);
-      const float dy = (float)(back >> 4) - (float)(t >> 4);
-      const bool mask_cycle = (sqrtf(dx * dx + dy * dy) <= p.patch_threshold) && (tail.cmax[ridx] >= thr);
-      // reference quirk kept on purpose: `idx_src2tar != 0` is indexed by s but multiplied position-wise with t
-      float mnz = tm * tail.smask[ridx];
-      mnz = mnz * (tail.cidx[t] != 0 ? 1.0f : 0.0f);
-      mnz = mnz * (ridx != 0 ? 1.0f : 0.0f);
-      const float mall = (mask_sim && mask_cycle) ? mnz : 0.0f;
-      float s_contrib = rmax * mall, s_mall = mall;
-#pragma unroll
-      for (int off = 16; off > 0; off >>= 1) {
-        s_contrib += __shfl_xor_sync(0xffffffffu, s_contrib, off);
-        s_mall += __shfl_xor_sync(0xffffffffu, s_mall, off);
-      }
-      if (lane == 0) { tail.red[0][e] = s_contrib; tail.red[1][e] = s_mall; }
-      p.rec_score[rec * kP + t] = rmax;
-      p.rec_idx[rec * kP + t] = (uint8_t)ridx;
-      p.rec_valid[rec * kP + t] = (mall != 0.0f) ? 1 : 0;
-      named_barrier_sync(1, kEpiThreads);
-      if (t == 0) {
-        float a = 0.f, m = 0.f;
-#pragma unroll
-        for (int g = 0; g < kEpiWarps; ++g) { a += tail.red[0][g]; m += tail.red[1][g]; }
-        p.sim_avg[rec] = (m > 0.f) ? a / (float)kP : 0.0f;              // matching.py:274-278
-      }
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, kTmemCols);
-  }
-}
-
-// ------------------------------------------------------------------------------------------------------------
-// CTA-pair form (2-CTA cluster on the two SMs of a TPC, tcgen05 cta_group::2): one item = ONE M=256 x N=256 UMMA
-// stream.  CTA r of the pair owns the query rows t in [128r, 128r+128) and stages HALF of the template slab (s rows
-// [128r, 128r+128)); the leader issues the instructions, which read both CTAs' shared memory, and every CTA drains
-// its own 128 accumulator rows.  Against the 1-CTA kernel the template planes are streamed from L2 / HBM once per item
-// instead of once per t-half (at one query per object that second read missed L2: 1.6x the algorithmic DRAM traffic),
-// and each SM's tensor core reads 4 KB + 4 KB of operands per instruction instead of 4 KB + 8 KB.
-// The column maxima (idx_src2tar: arg-max over ALL 256 query patches) of the two halves are exchanged through
-// distributed shared memory (st.shared::cluster + mbarrier release / acquire at cluster scope); the per-template score
-// is summed by the leader in the same order as the 1-CTA kernel (bit-identical results).
-// ------------------------------------------------------------------------------------------------------------
-namespace {
 constexpr int kPairStages = 6;
 constexpr int kPairStageBytes = 4 * kQPlaneBytes;            // q_hi, q_lo, t_hi half, t_lo half: 32 KB
 constexpr uint32_t kIdescPair = umma_idesc_f16(256, 256, /*bf16*/ 1);
@@ -564,7 +298,7 @@ sim_search_pair_kernel(const __grid_constant__ CUtensorMap tm_q_hi, const __grid
         p.rec_idx[rec * kP + t] = (uint8_t)ri;
         p.rec_valid[rec * kP + t] = (mall != 0.0f) ? 1 : 0;
       }
-      if (e < 4) {                             // warps 0..3 hold the patches: same lanes / order as warp 4 rank + e of the 1-CTA kernel
+      if (e < 4) {                             // epilogue warps 0..3 hold the patches: red[] lists the 8 sums in ascending t
 #pragma unroll
         for (int off = 16; off > 0; off >>= 1) {
           s_contrib += __shfl_xor_sync(0xffffffffu, s_contrib, off);
@@ -736,31 +470,15 @@ cudaError_t launch_sim_search(const CUtensorMap& q_hi, const CUtensorMap& q_lo, 
                               const CUtensorMap& t_lo, const SimSearchParams& p, int num_sms, cudaStream_t stream) {
   static bool configured = false;
   if (!configured) {
-    cudaError_t e = cudaFuncSetAttribute(sim_search_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(sim_search_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(sim_search_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPairSmemBytes);
+    cudaError_t e = cudaFuncSetAttribute(sim_search_pair_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPairSmemBytes);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(sim_search_pair_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kPairSmemBytes);
     if (e != cudaSuccess) return e;
     configured = true;
   }
   if (p.num_items <= 0) return cudaSuccess;
-  if (p.pair) {                                   // one 2-CTA cluster per item; t_hi / t_lo must be the 128-row-box maps
-    const int clusters = p.num_items < num_sms / 2 ? p.num_items : num_sms / 2;
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(2 * clusters); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = kPairSmemBytes; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    if (p.debug_tile) return cudaLaunchKernelEx(&cfg, sim_search_pair_kernel<true>, q_hi, q_lo, t_hi, t_lo, p);
-    return cudaLaunchKernelEx(&cfg, sim_search_pair_kernel<false>, q_hi, q_lo, t_hi, t_lo, p);
-  }
-  const int grid = p.num_items < num_sms ? p.num_items : num_sms;
-  if (p.debug_tile)
-    sim_search_kernel<true><<<grid, kThreads, kSmemBytes, stream>>>(q_hi, q_lo, t_hi, t_lo, p);
-  else
-    sim_search_kernel<false><<<grid, kThreads, kSmemBytes, stream>>>(q_hi, q_lo, t_hi, t_lo, p);
-  return cudaGetLastError();
+  const int clusters = p.num_items < num_sms / 2 ? p.num_items : num_sms / 2;   // one 2-CTA cluster per item
+  auto kernel = p.debug_tile ? sim_search_pair_kernel<true> : sim_search_pair_kernel<false>;
+  return launch_ex(kernel, dim3(2 * clusters), dim3(kThreads), kPairSmemBytes, stream, 2, q_hi, q_lo, t_hi, t_lo, p);
 }
 
 cudaError_t launch_topk_select(const TopkSelectParams& p, cudaStream_t stream) {
@@ -775,6 +493,6 @@ cudaError_t launch_topk_merge_expand(const TopkMergeParams& p, cudaStream_t stre
   return cudaGetLastError();
 }
 
-int sim_search_smem_bytes() { return kSmemBytes > kPairSmemBytes ? kSmemBytes : kPairSmemBytes; }
+int sim_search_smem_bytes() { return kPairSmemBytes; }
 
 }  // namespace gp

@@ -7,7 +7,6 @@
 
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <new>
 #include <string>
 #include <vector>
@@ -30,7 +29,7 @@ struct Carver {
   template <typename T> T* take(size_t n) { T* p = base ? reinterpret_cast<T*>(base + off) : nullptr; off += up(n * sizeof(T)); return p; }
 };
 
-struct Planes { uint16_t *hi, *lo; CUtensorMap m_hi, m_lo; CUtensorMap p_hi, p_lo; /* weights: 128-row boxes for CTA pairs */ };
+struct Planes { uint16_t *hi, *lo; CUtensorMap m_hi, m_lo; };
 
 struct BlockW {
   Planes qkv, proj, fc1, fc2;
@@ -47,7 +46,6 @@ struct BlockW {
 
 struct gp_vit_context {
   int depth, max_crops, passes, num_sms;
-  int pair;                    // linears run as 2-CTA cluster tiles (tcgen05 cta_group::2)
   Planes patch_w;
   const float *patch_b, *cls, *pos;
   std::vector<BlockW> blocks;
@@ -86,10 +84,14 @@ void carve_workspace(Carver& c, int max_crops, gp_vit_context* h) {
 
 int make_maps(Planes* p, uint64_t rows, uint64_t cols, uint32_t box_rows) {
   if (int e = gp_internal_make_map(&p->m_hi, p->hi, rows, cols, box_rows)) return e;
-  if (int e = gp_internal_make_map(&p->m_lo, p->lo, rows, cols, box_rows)) return e;
-  if (box_rows != 256) return GP_OK;
-  if (int e = gp_internal_make_map(&p->p_hi, p->hi, rows, cols, 128)) return e;     // half tiles: one per CTA of a pair
-  return gp_internal_make_map(&p->p_lo, p->lo, rows, cols, 128);
+  return gp_internal_make_map(&p->m_lo, p->lo, rows, cols, box_rows);
+}
+
+// A linear layer runs on 2-CTA cluster tiles (tcgen05 cta_group::2, 256 x 256): each CTA of a pair stages 128 rows of
+// the activations and 128 rows of the weights, so both operands' maps have 128-row boxes.
+cudaError_t linear(const gp_vit_context* h, const Planes& a, const Planes& w, gp::GemmParams g, cudaStream_t s) {
+  g.pair = 1;
+  return gp::launch_vit_gemm(a.m_hi, a.m_lo, w.m_hi, w.m_lo, g, h->num_sms, s);
 }
 
 }  // namespace
@@ -124,10 +126,6 @@ int gp_vit_create(int device, int depth, int max_crops, int precision, const flo
   if (!h) return gp_internal_fail(GP_ERR_INVALID, "out of host memory");
   h->depth = depth; h->max_crops = max_crops; h->num_sms = prop.multiProcessorCount;
   h->passes = precision == GP_PRECISION_FP32_SPLIT ? 3 : 1;
-  {
-    const char* ev = getenv("GIGAPOSE_GEMM_PAIR");
-    h->pair = ev ? (ev[0] != '0') : 1;        // default on; GIGAPOSE_GEMM_PAIR=0 selects the 1-CTA 128 x 256 tiles
-  }
   h->blocks.resize(depth);
   Carver cw(weight_mem), cs(workspace_mem);
   carve_weights(cw, depth, h);
@@ -150,8 +148,8 @@ int gp_vit_create(int device, int depth, int max_crops, int precision, const flo
     if ((ce = gp::launch_split_planes(b[4], kDim, kDim, kDim, B.proj.hi, B.proj.lo, s)) != cudaSuccess) break;
     if ((ce = gp::launch_split_planes(b[9], kMlp, kDim, kDim, B.fc1.hi, B.fc1.lo, s)) != cudaSuccess) break;
     if ((ce = gp::launch_split_planes(b[11], kDim, kMlp, kMlp, B.fc2.hi, B.fc2.lo, s)) != cudaSuccess) break;
-    if ((e = make_maps(&B.qkv, kQkv, kDim, 256)) || (e = make_maps(&B.proj, kDim, kDim, 256)) ||
-        (e = make_maps(&B.fc1, kMlp, kDim, 256)) || (e = make_maps(&B.fc2, kDim, kMlp, 256)))
+    if ((e = make_maps(&B.qkv, kQkv, kDim, 128)) || (e = make_maps(&B.proj, kDim, kDim, 128)) ||
+        (e = make_maps(&B.fc1, kMlp, kDim, 128)) || (e = make_maps(&B.fc2, kDim, kMlp, 128)))
       break;
   }
   const uint64_t M = (uint64_t)max_crops * kTok;
@@ -196,27 +194,22 @@ int gp_vit_time_linears(gp_vit_handle_t h, int b, int iters, float* avg_ms, void
   if (b < 1 || b > h->max_crops) return gp_internal_fail(GP_ERR_INVALID, "batch %d outside [1, %d]", b, h->max_crops);
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   const int M = b * kTok;
-  auto linear = [&](const Planes& a, const Planes& w, gp::GemmParams& gp_) {
-    gp_.pair = h->pair;
-    return h->pair ? gp::launch_vit_gemm(a.m_hi, a.m_lo, w.p_hi, w.p_lo, gp_, h->num_sms, s)
-                   : gp::launch_vit_gemm(a.m_hi, a.m_lo, w.m_hi, w.m_lo, gp_, h->num_sms, s);
-  };
   auto run = [&]() -> int {
     for (int i = 0; i < h->depth; ++i) {
       const BlockW& B = h->blocks[i];
       gp::GemmParams g{};
       g.passes = h->passes; g.M = M; g.N = kQkv; g.K = kDim; g.mode = gp::GEMM_QKV_HEADS; g.bias = B.qkv_b;
       g.out_hi = h->qkv.hi; g.out_lo = h->qkv.lo; g.tokens_per_img = kTok; g.qkv_crop_stride = h->max_crops;
-      GPV_CUDA(linear(h->ln, B.qkv, g));
+      GPV_CUDA(linear(h, h->ln, B.qkv, g, s));
       g = gp::GemmParams{}; g.passes = h->passes;
       g.M = M; g.N = kDim; g.K = kDim; g.mode = gp::GEMM_SCALE_RESIDUAL; g.bias = B.proj_b; g.gamma = B.ls1; g.x = h->x;
-      GPV_CUDA(linear(h->attn, B.proj, g));
+      GPV_CUDA(linear(h, h->attn, B.proj, g, s));
       g = gp::GemmParams{}; g.passes = h->passes;
       g.M = M; g.N = kMlp; g.K = kDim; g.mode = gp::GEMM_PLANES_GELU; g.bias = B.fc1_b; g.out_hi = h->hid.hi; g.out_lo = h->hid.lo;
-      GPV_CUDA(linear(h->ln, B.fc1, g));
+      GPV_CUDA(linear(h, h->ln, B.fc1, g, s));
       g = gp::GemmParams{}; g.passes = h->passes;
       g.M = M; g.N = kDim; g.K = kMlp; g.mode = gp::GEMM_SCALE_RESIDUAL; g.bias = B.fc2_b; g.gamma = B.ls2; g.x = h->x;
-      GPV_CUDA(linear(h->hid, B.fc2, g));
+      GPV_CUDA(linear(h, h->hid, B.fc2, g, s));
     }
     return GP_OK;
   };
@@ -250,30 +243,25 @@ int gp_vit_forward(gp_vit_handle_t h, int b, const float* img, float* x_prenorm,
   g.M = b * 256; g.N = kDim; g.K = kPatchKPad; g.mode = gp::GEMM_PATCH_EMBED; g.bias = h->patch_b; g.pos = h->pos; g.x = h->x;
   GPV_CUDA(gp::launch_vit_gemm(h->patches.m_hi, h->patches.m_lo, h->patch_w.m_hi, h->patch_w.m_lo, g, h->num_sms, s));
   GPV_CUDA(gp::launch_cls_rows(h->cls, h->pos, b, h->x, s));
-  auto linear = [&](const Planes& a, const Planes& w, gp::GemmParams& gp_) {
-    gp_.pair = h->pair;
-    return h->pair ? gp::launch_vit_gemm(a.m_hi, a.m_lo, w.p_hi, w.p_lo, gp_, h->num_sms, s)
-                   : gp::launch_vit_gemm(a.m_hi, a.m_lo, w.m_hi, w.m_lo, gp_, h->num_sms, s);
-  };
   for (int i = 0; i < h->depth; ++i) {
     const BlockW& B = h->blocks[i];
     GPV_CUDA(gp::launch_layernorm_planes(h->x, M, B.n1w, B.n1b, 1e-6f, h->ln.hi, h->ln.lo, s));
     g = gp::GemmParams{}; g.passes = h->passes;
     g.M = M; g.N = kQkv; g.K = kDim; g.mode = gp::GEMM_QKV_HEADS; g.bias = B.qkv_b; g.out_hi = h->qkv.hi; g.out_lo = h->qkv.lo;
     g.tokens_per_img = kTok; g.qkv_crop_stride = h->max_crops;
-    GPV_CUDA(linear(h->ln, B.qkv, g));
+    GPV_CUDA(linear(h, h->ln, B.qkv, g, s));
     GPV_CUDA(gp::launch_attention_tc(h->qkv_hi128, h->qkv_lo128, h->qkv_hi16, h->qkv_lo16, h->qkv.hi, h->qkv.lo,
                                      h->attn.hi, h->attn.lo, b, h->max_crops, h->passes, s));
     g = gp::GemmParams{}; g.passes = h->passes;
     g.M = M; g.N = kDim; g.K = kDim; g.mode = gp::GEMM_SCALE_RESIDUAL; g.bias = B.proj_b; g.gamma = B.ls1; g.x = h->x;
-    GPV_CUDA(linear(h->attn, B.proj, g));
+    GPV_CUDA(linear(h, h->attn, B.proj, g, s));
     GPV_CUDA(gp::launch_layernorm_planes(h->x, M, B.n2w, B.n2b, 1e-6f, h->ln.hi, h->ln.lo, s));
     g = gp::GemmParams{}; g.passes = h->passes;
     g.M = M; g.N = kMlp; g.K = kDim; g.mode = gp::GEMM_PLANES_GELU; g.bias = B.fc1_b; g.out_hi = h->hid.hi; g.out_lo = h->hid.lo;
-    GPV_CUDA(linear(h->ln, B.fc1, g));
+    GPV_CUDA(linear(h, h->ln, B.fc1, g, s));
     g = gp::GemmParams{}; g.passes = h->passes;
     g.M = M; g.N = kDim; g.K = kMlp; g.mode = gp::GEMM_SCALE_RESIDUAL; g.bias = B.fc2_b; g.gamma = B.ls2; g.x = h->x;
-    GPV_CUDA(linear(h->hid, B.fc2, g));
+    GPV_CUDA(linear(h, h->hid, B.fc2, g, s));
   }
   GPV_CUDA(cudaMemcpyAsync(x_prenorm, h->x, (size_t)M * kDim * sizeof(float), cudaMemcpyDeviceToDevice, s));
   gp_internal_count_launches(3 + 7 * h->depth);

@@ -82,7 +82,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tm_hi_128, const __grid_
                     __nv_bfloat16* __restrict__ out_hi, __nv_bfloat16* __restrict__ out_lo, int crop_stride, int num_items) {
   constexpr int passes = kPasses;
   extern __shared__ uint8_t smem_raw[];
-  pdl_trigger();
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint8_t* sK[2] = {smem, smem + kKVPlane};                                   // hi, lo
   uint8_t* sV[2] = {smem + 2 * kKVPlane, smem + 3 * kKVPlane};
@@ -115,7 +114,6 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tm_hi_128, const __grid_
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = tail.tmem_base;
-  pdl_wait();                                        // q / k / v planes come from the QKV GEMM launched before
   if (threadIdx.x == 0) STAMP(0);
 
   if (warp == 0) {
@@ -459,8 +457,8 @@ cudaError_t launch_attention_tc(const CUtensorMap& hi128, const CUtensorMap& lo1
   auto qh = reinterpret_cast<const __nv_bfloat16*>(qkv_hi), ql = reinterpret_cast<const __nv_bfloat16*>(qkv_lo);
   auto oh = reinterpret_cast<__nv_bfloat16*>(out_hi), ol = reinterpret_cast<__nv_bfloat16*>(out_lo);
   if (passes == 3)
-    return launch_ex(attention_tc_kernel<3>, grid, dim3(kThreads), kSmem, s, 1, true, hi128, lo128, hi16, lo16, qh, ql, oh, ol, crop_stride, items);
-  return launch_ex(attention_tc_kernel<1>, grid, dim3(kThreads), kSmem, s, 1, true, hi128, lo128, hi16, lo16, qh, ql, oh, ol, crop_stride, items);
+    return launch_ex(attention_tc_kernel<3>, grid, dim3(kThreads), kSmem, s, 1, hi128, lo128, hi16, lo16, qh, ql, oh, ol, crop_stride, items);
+  return launch_ex(attention_tc_kernel<1>, grid, dim3(kThreads), kSmem, s, 1, hi128, lo128, hi16, lo16, qh, ql, oh, ol, crop_stride, items);
 }
 
 }  // namespace gp

@@ -12,9 +12,9 @@
 //   warps 4-11 epilogue    (TMEM -> registers -> fused bias / GELU / ReLU / LayerScale + residual / shortcut /
 //                           positional table -> fp32 rows or bf16 hi/lo planes for the next layer), overlapping the
 //                           next tile's MMAs; stores are transposed through shared memory into full 64-byte segments.
-// Three instantiations: <swap=0,pair=0> 128 x bn tiles on one CTA; <0,1> 256 x bn tiles on a 2-CTA cluster
-// (tcgen05 cta_group::2, the ViT linears); <1,0> filters as the 128-row operand against 256 output pixels (the
-// 128-channel convolutions).
+// Three tile shapes: <swap=0,pair=0> 128 x bn tiles on one CTA (patch embedding, convolutions); <0,1> 256 x bn tiles on
+// a 2-CTA cluster (tcgen05 cta_group::2: the ViT linears and the IST regressor's hidden layers); <1,0> filters as the
+// 128-row operand against 256 output pixels (the 128-channel convolutions).
 #include "gigapose_kernels.h"
 #include "common.cuh"
 #include <cuda_bf16.h>
@@ -105,7 +105,6 @@ __global__ void __launch_bounds__(kThreads, 1)
 vit_gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
                 const __grid_constant__ CUtensorMap tm_w_hi, const __grid_constant__ CUtensorMap tm_w_lo, GemmParams p) {
   extern __shared__ uint8_t smem_raw[];
-  pdl_trigger();                                     // the next kernel's CTAs may take SMs as this grid's CTAs retire
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   static_assert(!(kSwap && kPair), "the swapped layers have M = 128 filters: nothing to pair");
   constexpr int kNumStages = kPair ? kPairStages : kStages;
@@ -143,7 +142,6 @@ vit_gemm_kernel(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_consta
   if constexpr (kPair) cluster_sync_all();         // barriers and TMEM of the peer exist before anything reaches across
   tc_fence_after();
   const uint32_t tmem_base = tail.tmem_base;
-  pdl_wait();                                        // everything above overlapped the previous kernel's tail
   if (threadIdx.x == 0) GSTAMP(63);
 
   if (warp == 0) {
@@ -492,7 +490,7 @@ cudaError_t launch_mode(const CUtensorMap& a_hi, const CUtensorMap& a_lo, const 
     if (e != cudaSuccess) return e;
     configured = true;
   }
-  return launch_ex(vit_gemm_kernel<kSwap, kPair, kMode>, dim3(grid), dim3(kThreads), kSmemBytes, stream, cluster, true, a_hi, a_lo,
+  return launch_ex(vit_gemm_kernel<kSwap, kPair, kMode>, dim3(grid), dim3(kThreads), kSmemBytes, stream, cluster, a_hi, a_lo,
                    w_hi, w_lo, p);
 }
 }  // namespace
@@ -504,9 +502,10 @@ cudaError_t launch_vit_gemm(const CUtensorMap& a_hi, const CUtensorMap& a_lo, co
   if ((bn != 128 && bn != 192 && bn != 256) || p.N % bn != 0 || p.K % kBlockK != 0) return cudaErrorInvalidValue;
   const int tile_pixels = p.swap ? bn : kBM;
   if (p.conv && (p.Wo <= 0 || tile_pixels % p.Wo != 0 || p.M % kBM != 0 || p.cblocks <= 0)) return cudaErrorInvalidValue;
-  if (p.swap && (p.pair || bn != kBN || p.M % kBM != 0 ||
-                 (p.mode != GEMM_PLANES && p.mode != GEMM_PLANES_RELU && p.mode != GEMM_PLANES_ADD_RELU)))
-    return cudaErrorInvalidValue;
+  if (p.swap && (p.pair || bn != kBN || p.M % kBM != 0)) return cudaErrorInvalidValue;
+  // Only the mode / tile-shape combinations some caller launches are instantiated; any other returns
+  // cudaErrorInvalidValue.  Pairs: the ViT linears (vit_api.cu) and the IST regressor's hidden layers (api.cu).  1-CTA
+  // tiles: the patch embedding and the IST trunk's convolutions (ist_trunk.cu), swapped for the 128-channel layers.
 #define GP_GEMM_CASE(SWAP, PAIR, MODE) \
   case MODE: return launch_mode<SWAP, PAIR, MODE>(a_hi, a_lo, w_hi, w_lo, p, grid, PAIR ? 2 : 1, stream);
   if (p.pair) {                                   // one 2-CTA cluster per 256 x bn tile
@@ -518,9 +517,6 @@ cudaError_t launch_vit_gemm(const CUtensorMap& a_hi, const CUtensorMap& a_lo, co
       GP_GEMM_CASE(false, true, GEMM_SCALE_RESIDUAL)
       GP_GEMM_CASE(false, true, GEMM_PLANES_GELU)
       GP_GEMM_CASE(false, true, GEMM_PLANES_RELU)
-      GP_GEMM_CASE(false, true, GEMM_PLANES_ADD_RELU)
-      GP_GEMM_CASE(false, true, GEMM_PLANES)
-      GP_GEMM_CASE(false, true, GEMM_ROWS_F32)
       GP_GEMM_CASE(false, true, GEMM_ROWS_F32_RELU)
       default: return cudaErrorInvalidValue;
     }
@@ -529,7 +525,6 @@ cudaError_t launch_vit_gemm(const CUtensorMap& a_hi, const CUtensorMap& a_lo, co
   const int grid = tiles < num_sms ? tiles : num_sms;
   if (p.swap) {
     switch (p.mode) {
-      GP_GEMM_CASE(true, false, GEMM_PLANES)
       GP_GEMM_CASE(true, false, GEMM_PLANES_RELU)
       GP_GEMM_CASE(true, false, GEMM_PLANES_ADD_RELU)
       default: return cudaErrorInvalidValue;
@@ -537,14 +532,10 @@ cudaError_t launch_vit_gemm(const CUtensorMap& a_hi, const CUtensorMap& a_lo, co
   }
   switch (p.mode) {
     GP_GEMM_CASE(false, false, GEMM_PLANES)
-    GP_GEMM_CASE(false, false, GEMM_PLANES_GELU)
-    GP_GEMM_CASE(false, false, GEMM_SCALE_RESIDUAL)
     GP_GEMM_CASE(false, false, GEMM_PATCH_EMBED)
-    GP_GEMM_CASE(false, false, GEMM_QKV_HEADS)
     GP_GEMM_CASE(false, false, GEMM_PLANES_RELU)
     GP_GEMM_CASE(false, false, GEMM_PLANES_ADD_RELU)
     GP_GEMM_CASE(false, false, GEMM_ROWS_F32)
-    GP_GEMM_CASE(false, false, GEMM_ROWS_F32_RELU)
     default: return cudaErrorInvalidValue;
   }
 #undef GP_GEMM_CASE

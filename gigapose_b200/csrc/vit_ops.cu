@@ -2,7 +2,6 @@
 // (-> bf16 hi/lo planes, the A operand of the next tcgen05 GEMM) and the fp32 -> hi/lo plane split used to pack weights.
 // Attention lives in vit_attention_tc.cu.
 #include "gigapose_kernels.h"
-#include "common.cuh"
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 
@@ -63,8 +62,6 @@ __global__ void im2col_kernel(const float* __restrict__ img, int b, int Kpad, __
 
 // ---------------------------------------------------------------- x[b*257 + 0, :] = cls + pos[0]
 __global__ void cls_rows_kernel(const float* __restrict__ cls, const float* __restrict__ pos, int b, float* __restrict__ x) {
-  pdl_trigger();
-  pdl_wait();
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= b * kDim) return;
   const int im = i / kDim, c = i - im * kDim;
@@ -75,10 +72,8 @@ __global__ void cls_rows_kernel(const float* __restrict__ cls, const float* __re
 __global__ void __launch_bounds__(256)
 layernorm_planes_kernel(const float* __restrict__ x, int M, const float* __restrict__ w, const float* __restrict__ bsh,
                         float eps, __nv_bfloat16* __restrict__ hi, __nv_bfloat16* __restrict__ lo) {
-  pdl_trigger();
   const int row = blockIdx.x * 8 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
-  pdl_wait();
   if (row >= M) return;
   const float4* src = reinterpret_cast<const float4*>(x + (size_t)row * kDim);
   float4 v[8];
@@ -146,13 +141,13 @@ cudaError_t launch_im2col(const float* img, int b, int Kpad, uint16_t* hi, uint1
 
 cudaError_t launch_cls_rows(const float* cls, const float* pos, int b, float* x, cudaStream_t s) {
   if (b <= 0) return cudaSuccess;
-  return launch_ex(cls_rows_kernel, dim3((b * kDim + 255) / 256), dim3(256), 0, s, 1, true, cls, pos, b, x);
+  return launch_ex(cls_rows_kernel, dim3((b * kDim + 255) / 256), dim3(256), 0, s, 1, cls, pos, b, x);
 }
 
 cudaError_t launch_layernorm_planes(const float* x, int M, const float* w, const float* b, float eps, uint16_t* hi,
                                     uint16_t* lo, cudaStream_t s) {
   if (M <= 0) return cudaSuccess;
-  return launch_ex(layernorm_planes_kernel, dim3((M + 7) / 8), dim3(256), 0, s, 1, true, x, M, w, b, eps,
+  return launch_ex(layernorm_planes_kernel, dim3((M + 7) / 8), dim3(256), 0, s, 1, x, M, w, b, eps,
                    reinterpret_cast<__nv_bfloat16*>(hi), reinterpret_cast<__nv_bfloat16*>(lo));
 }
 

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Similarity kernel at the per-GPU shard of BASELINE.json configs[4] (stress: 256 objects x 576 templates over 8 GPUs
 = 72 local templates per object, batch 256, ONE query per object -> no template reuse, B_o = 1): reports the achieved
-HBM GB/s and TFLOP/s of `sim_search_kernel` in both precisions.  Feature-level synthetic data generated on the device.
+HBM GB/s and TFLOP/s of `sim_search_pair_kernel` in both precisions.  Feature-level synthetic data generated on the device.
 
     python scripts/stress_sim.py [--objects 256] [--templates 72] [--out gpurun_out/stress_sim.json]
 """
@@ -32,8 +32,7 @@ def main():
     res = {"workload": f"per-GPU shard of c5: {O} objects x {T} local templates, batch {B}, one query per object",
            "bank_GB": O * T * 256 * 1024 * 4 / 1e9}
     labels = torch.arange(1, O + 1)
-    for prec, pair in (("fp32_split", 0), ("fp32_split", 1), ("bf16", 0), ("bf16", 1)):
-        os.environ["GIGAPOSE_SIM_PAIR"] = str(pair)          # read when the handle is created
+    for prec in ("fp32_split", "bf16"):
         eng = Engine(O, T, B, device=dev, precision=prec)
         # generate + load the bank object-chunk by object-chunk (keeps the fp32 staging copy small)
         q_feat = None
@@ -54,7 +53,7 @@ def main():
         plane_bytes = 4 if passes == 3 else 2                      # bf16 mode streams the hi planes only
         alg_bytes = O * T * 256 * 1024 * plane_bytes + B * 256 * 1024 * plane_bytes + B * T * (256 * 6 + 4)
         flops = 2.0 * B * T * 256 * 256 * 1024
-        res[f"{prec}_{'pair' if pair else '1cta'}"] = {"ms_per_launch": ms, "kernel": "sim_search_pair_kernel (2-CTA cluster)" if pair else "sim_search_kernel", "algorithmic_GB": alg_bytes / 1e9, "achieved_GBps": alg_bytes / (ms / 1e3) / 1e9,
+        res[prec] = {"ms_per_launch": ms, "kernel": "sim_search_pair_kernel (2-CTA cluster)", "algorithmic_GB": alg_bytes / 1e9, "achieved_GBps": alg_bytes / (ms / 1e3) / 1e9,
                      "hbm_peak_GBps": peaks.get("hbm_gbs"), "hbm_frac": alg_bytes / (ms / 1e3) / 1e9 / peaks.get("hbm_gbs", 6650.0),
                      "algorithmic_TFLOPs": flops / (ms / 1e3) / 1e12, "executed_TFLOPs": passes * flops / (ms / 1e3) / 1e12,
                      "bf16_peak_TFLOPs": peaks.get("bf16_tflops"), "detections_per_s_sim_only": B / (ms / 1e3),

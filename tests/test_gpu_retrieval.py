@@ -10,7 +10,7 @@ import torch.nn.functional as F
 from gigapose_b200 import synth
 from oracle import port
 
-from helpers import FLOAT_KEYS, INT_KEYS, cpu, engine_from_case, run_engine
+from helpers import FLOAT_KEYS, INT_KEYS, cpu, engine_from_case, reference_slice, run_engine, write_report
 
 pytestmark = pytest.mark.gpu
 
@@ -23,12 +23,17 @@ def _ref_tiles(case, dtype=torch.float64):
     return torch.einsum("btc,bnsc->nbts", q, bank)
 
 
-@pytest.mark.parametrize("precision,tol", [("fp32_split", 1e-5), ("bf16", 2e-2)])
-def test_similarity_tiles_against_fp64(precision, tol):
+@pytest.mark.parametrize("precision,tol,B,O,T,seed", [
+    pytest.param("fp32_split", 1e-5, 3, 2, 6, 3, id="fp32_split-1e-05"),
+    pytest.param("bf16", 2e-2, 3, 2, 6, 3, id="bf16-0.02"),
+    pytest.param("fp32_split", 1e-5, 5, 2, 10, 82, id="fp32_split-1e-05-5x2x10"),
+    pytest.param("fp32_split", 1e-5, 3, 3, 5, 80, id="fp32_split-1e-05-3x3x5"),
+])
+def test_similarity_tiles_against_fp64(precision, tol, B, O, T, seed):
     """The TMA + tcgen05 main loop alone: raw fp32 tiles vs an fp64 einsum on the same descriptors.
     fp32_split measures ~4e-6 (the tensor core adds into its fp32 accumulator with truncation, 192 adds per
     element); the reference's own fp32 einsum sits at ~1e-7, plain bf16 at ~5e-3."""
-    case = synth.make_feature_case(B=3, O=2, T=6, seed=3)
+    case = synth.make_feature_case(B=B, O=O, T=T, seed=seed)
     eng = engine_from_case(case, precision=precision)
     eng.set_queries(case.q_feat, case.q_mask16.reshape(-1, 16, 16), case.q_label - 1)
     tiles = eng.debug_sim_tiles().cpu().double()
@@ -144,58 +149,55 @@ def test_empty_and_degenerate_queries():
         assert torch.equal(out[k][[0, 2]].to(ref[k].dtype), ref[k][[0, 2]]), k
 
 
-@pytest.mark.parametrize("B,O,T", [(5, 2, 10), (3, 3, 1), (32, 8, 162)])
-def test_pair_kernel_equals_the_one_cta_kernel(B, O, T, monkeypatch):
-    """`sim_search_pair_kernel` (2-CTA clusters, tcgen05 cta_group::2, column maxima exchanged through distributed
-    shared memory; the default) against `sim_search_kernel` (GIGAPOSE_SIM_PAIR=0): every integer output of the chain is
-    equal; floats agree to fp32 accumulation-order noise (the 1-CTA kernel walks the k-blocks of its second t-half
-    backwards, the pair kernel walks all of them forwards, so rows t >= 128 round differently in the last bit)."""
-    case = synth.make_feature_case(B=B, O=O, T=max(T, 5), seed=77 + B)
-    reg = port.RegressorPort(seed=6)
-    outs = []
-    for pair in ("0", "1"):
-        monkeypatch.setenv("GIGAPOSE_SIM_PAIR", pair)
-        eng = engine_from_case(case, regressor=reg)
-        out = cpu(run_engine(eng, case))
-        eng.set_queries(case.q_feat, case.q_mask16.reshape(-1, 16, 16), case.q_label - 1)
-        cand = cpu(eng.sim_candidates())
-        out.update({"cand_" + k: v for k, v in cand.items()})
-        if B <= 8:
-            out["tiles"] = eng.debug_sim_tiles().cpu()
-        outs.append(out)
-    for k in outs[0]:
-        a, b = outs[0][k], outs[1][k]
-        if a.dtype.is_floating_point:
-            finite = torch.isfinite(a) & torch.isfinite(b)
-            assert torch.equal(torch.isfinite(a), torch.isfinite(b)), k
-            tol = 2e-3 if k in ("M", "pred_poses") else 5e-6
-            assert torch.allclose(a[finite], b[finite], atol=tol, rtol=1e-5), (k, float((a[finite] - b[finite]).abs().max()))
-        else:
-            assert torch.equal(a, b), k
+@pytest.mark.parametrize("B,O,T", [(5, 2, 10), (3, 3, 5), (32, 8, 162)])
+def test_pair_kernel_against_oracle(B, O, T):
+    """Row a4 (`sim_search_pair_kernel`: 2-CTA clusters, tcgen05 cta_group::2, column maxima exchanged through
+    distributed shared memory) against the CPU oracle for every detection: template ids and correspondences bit-exact,
+    scores within 2e-6.  The oracle is fed a few detections at a time (the full c2 reference layout is ~5 GB)."""
+    case = synth.make_feature_case(B=B, O=O, T=T, seed=77 + B)
+    eng = engine_from_case(case)
+    eng.set_queries(case.q_feat, case.q_mask16.reshape(-1, 16, 16), case.q_label - 1)
+    m = cpu(eng.sim_topk())
+    for b0 in range(0, B, 4):
+        sel = torch.arange(b0, min(B, b0 + 4))
+        ri = reference_slice(case, sel)
+        sim = port.similarity_search(ri["src_feats"], ri["tar_feat"], ri["src_masks"], ri["tar_mask"])
+        for k in ("id_src", "tar_pts", "src_pts"):
+            assert torch.equal(m[k][sel], sim[k]), (k, b0)
+        assert torch.allclose(m["score_src"][sel], sim["score_src"], atol=2e-6), b0
+        assert torch.allclose(m["score_pts"][sel], sim["score_pts"], atol=2e-6), b0
 
 
-def test_tensor_core_mlp_keeps_every_integer_output(monkeypatch):
-    """Row a5 on tcgen05 (split-bf16 x3 hidden layers through vit_gemm_kernel, fp32 heads; the default) against the fp32
-    SIMT kernels (GIGAPOSE_MLP_SIMT=1) on the c2-sized planted case: regressor outputs agree to 1e-4 and every integer
-    output downstream (inlier sets, failure flags, the re-sort) is unchanged."""
+def test_tensor_core_mlp_against_oracle():
+    """Row a5 on tcgen05 (fp16 hi/lo x3 hidden layers through vit_gemm_kernel, fp32 heads) against the fp32 oracle on
+    the c2-sized planted case and the engine's own matches: the -1000 pattern is identical, regressor outputs agree to
+    5e-5, and RANSAC + sort + pose on the GPU give the same integer outputs and scores with either set of outputs."""
     case = synth.make_feature_case(B=32, O=8, T=162, seed=42)
     reg = port.RegressorPort(seed=9)
-    outs = []
-    for simt in ("1", "0"):
-        monkeypatch.setenv("GIGAPOSE_MLP_SIMT", simt)
-        eng = engine_from_case(case, regressor=reg)
-        outs.append(cpu(run_engine(eng, case)))
-    a, b = outs
-    valid = a["src_pts"][..., 0] != -1
-    assert torch.equal(a["relScale"] == -1000, b["relScale"] == -1000)
-    d = max(float((a["relScale"] - b["relScale"])[valid].abs().max()), float((a["relInplane"] - b["relInplane"])[valid].abs().max()))
+    eng = engine_from_case(case, regressor=reg)
+    eng.set_queries(case.q_feat, case.q_mask16.reshape(-1, 16, 16), case.q_label - 1)
+    m = eng.sim_topk()
+    rs, ri = eng.ist_mlp(case.q_ist, m)
+    mc = cpu(m)
+    src_ist = case.bank_ist[(case.q_label - 1)[:, None], mc["id_src"]]          # [B,k,...] template IST features
+    rs_ref, ri_ref = torch.zeros(rs.shape), torch.zeros(ri.shape)
+    for kk in range(mc["id_src"].shape[1]):
+        rs_ref[:, kk], ri_ref[:, kk] = port.ist_mlp(reg, src_ist[:, kk], case.q_ist, mc["src_pts"][:, kk], mc["tar_pts"][:, kk])
+    rs_gpu, ri_gpu = rs.cpu(), ri.cpu()
+    valid = mc["src_pts"][..., 0] != -1
+    assert torch.equal(rs_gpu == -1000, rs_ref == -1000)
+    assert torch.equal(ri_gpu == -1000, ri_ref == -1000)
+    d = max(float((rs_gpu - rs_ref)[valid].abs().max()), float((ri_gpu - ri_ref)[valid].abs().max()))
+    dev = eng.device
+    a = cpu(eng.sort_and_pose(case.q_K, case.q_M, m, rs, ri, eng.ransac(m, rs, ri)))
+    rs_ref, ri_ref = rs_ref.to(dev), ri_ref.to(dev)
+    b = cpu(eng.sort_and_pose(case.q_K, case.q_M, m, rs_ref, ri_ref, eng.ransac(m, rs_ref, ri_ref)))
     perr = (a["pred_poses"] - b["pred_poses"]).abs()
-    perr[..., :3, 3] /= a["pred_poses"][..., :3, 3].abs().clamp(min=1.0)
-    from helpers import write_report
-    write_report("mlp_tc_vs_simt.json", {"case": "c2 planted features (32 detections, 8 x 162 templates)", "hypotheses": 160,
-                                         "valid_correspondences": int(valid.sum()), "regressor_output_max_abs_diff": d,
-                                         "pose_max_diff": float(perr.max()),
-                                         "integer_outputs_changed": int(sum((a[k] != b[k]).sum() for k in INT_KEYS))})
+    perr[..., :3, 3] /= b["pred_poses"][..., :3, 3].abs().clamp(min=1.0)
+    write_report("mlp_tc_vs_oracle.json", {"case": "c2 planted features (32 detections, 8 x 162 templates)", "hypotheses": 160,
+                                           "valid_correspondences": int(valid.sum()), "regressor_output_max_abs_diff": d,
+                                           "pose_max_diff": float(perr.max()),
+                                           "integer_outputs_changed": int(sum((a[k] != b[k]).sum() for k in INT_KEYS))})
     assert d < 5e-5, d
     assert float(perr.max()) < 1e-3
     for k in INT_KEYS:
